@@ -60,7 +60,37 @@ def parse():
                          "inside the library (not validated on hardware this round)")
     ap.add_argument("--merge-timeout", type=int, default=360, help="seconds after which a stalled mode B leg is abandoned (the headline line is printed without it)")
     ap.add_argument("--config", type=int, default=2, choices=[2, 3], help="BASELINE.json config: 2 = headline (default), 3 = Zipf/CUDA-origin/50k labelsets")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (the Arrow IPC stream and the batch "
+                    "counts) to DIR as .npy files, for comparing two builds output for output (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.stream or args.config4_local or args.config4_single):
+        ap.error("--dump-outputs covers the headline pass and --impl reference, not --stream or --config4-*")
+    return args
+
+
+DUMP_BYTES = 8 << 20  # stream bytes kept in ipc.npy per run (32 MB as float32)
+DUMP_BLOCK = 1 << 20
+
+
+def dump_outputs(path, ipc, counts, rank=0, world=1):
+    """Writes one pass's output as float .npy files: ipc = bytes of the IPC stream (all of it up to DUMP_BYTES, otherwise one
+    byte from each of DUMP_BYTES equal strides at offsets drawn from a fixed seed, so equal streams give equal samples),
+    ipc_block_sums = the byte sum of every DUMP_BLOCK bytes of the whole stream, counts = [rows, unique stacks, locations,
+    functions, location indices, stream bytes]. With several ranks each writes <name>_rank<r>.npy and keeps 1/world of the sample."""
+    ipc = np.frombuffer(ipc, dtype=np.uint8)
+    n, k = len(ipc), DUMP_BYTES // world
+    if n > k:
+        ipc_sample = ipc[np.arange(k, dtype=np.int64) * n // k + np.random.default_rng(0).integers(0, n // k, k)]
+    else:
+        ipc_sample = ipc
+    sums = np.add.reduceat(ipc, np.arange(0, n, DUMP_BLOCK), dtype=np.uint64) if n else np.zeros(0, np.uint64)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "ipc%s.npy" % suffix), ipc_sample.astype(np.float32))
+    np.save(os.path.join(path, "ipc_block_sums%s.npy" % suffix), sums.astype(np.float64))
+    np.save(os.path.join(path, "counts%s.npy" % suffix), np.array(list(counts) + [n], dtype=np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -141,7 +171,7 @@ def time_cpu_port(w, n_rows, keep_bytes=False):
     if keep_bytes:
         import hashlib
         st["ipc_sha256"] = hashlib.sha256(data).hexdigest()
-    return sub.n / dt, dt, len(data), st
+    return sub.n / dt, dt, data, st
 
 
 def two_core_note(n, st):
@@ -162,24 +192,24 @@ def run_reference(args, rank, world):
     n = w.n if args.ref_sample <= 0 else min(w.n, args.ref_sample)
     for _ in range(args.warmup):
         time_cpu_port(w, min(w.n, 100_000))
-    times, st, digest = [], None, None
-    budget_s = float(os.environ.get("PA_REF_BUDGET_S", "600"))  # a step is ~15 s of CPU (the driver asks for 20: ~5 min); a much slower host stops early and says so
+    times, st, digest, data = [], None, None, None
     for i in range(args.steps):
-        if times and float(np.sum(times)) + float(np.mean(times)) > budget_s:
-            break
-        rate, dt, nbytes, st = time_cpu_port(w, n, keep_bytes=(i == 0))
+        data = None  # the previous step's stream is not kept alive while the next one is timed
+        rate, dt, data, st = time_cpu_port(w, n, keep_bytes=(i == 0))
         digest = st.get("ipc_sha256", digest)
         times.append(dt)
+    if args.dump_outputs:  # rank 0's file names and sample positions, as the b200 arm writes them
+        from oracle.oracle_py import STAT_NAMES
+        dump_outputs(args.dump_outputs, data, [st[k] for k in STAT_NAMES[:5]], 0, world)
     total = float(np.sum(times))
-    steps_done = len(times)
-    value = n * steps_done / total
-    sample = ("%d rows per step = %s config-%d batch of one GPU, ingest+flush to IPC bytes, %d of the %d requested steps in %.0f s (every step is the "
-              "same deterministic pass; the run stops at a %.0f s budget); C++ restatement of the reference "
+    value = n * args.steps / total
+    sample = ("%d rows per step = %s config-%d batch of one GPU, ingest+flush to IPC bytes, %d steps in %.0f s (every step is the "
+              "same deterministic pass); C++ restatement of the reference "
               "Go path (Go toolchain unavailable), single thread as the reference serialises ingest (parca_reporter.go:335); host has %d cores"
-              % (n, "the whole" if n == w.n else "a prefix of the", args.config, steps_done, args.steps, total, budget_s, os.cpu_count()))
+              % (n, "the whole" if n == w.n else "a prefix of the", args.config, args.steps, total, os.cpu_count()))
     print(json.dumps({
         "impl": "reference", "metric": "samples/sec aggregated", "value": value, "unit": "samples/s", "n_gpus": args.gpus,
-        "steps": steps_done, "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * total / steps_done, "higher_is_better": True,
+        "steps": args.steps, "steps_requested": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * total / args.steps, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "u64", "data": "synthetic",
         "config": config_of(args, w, world),
         "cpu_baseline": {"value": value, "unit": "samples/s", "cores": 1, "kind": "port", "sample": sample, **two_core_note(n, st)},
@@ -560,6 +590,9 @@ def main():
     barrier()
     wall = time.perf_counter() - t0
     res = a.collect()
+    if args.dump_outputs:  # res.ipc is only valid until the next flush
+        dump_outputs(args.dump_outputs, res.ipc, [res.n_rows, res.n_unique_stacks, res.n_locations, res.n_functions, res.n_location_indices],
+                     rank, world)
     dev_s = float(np.sum(step_ms)) / 1e3
     tmax = torch.tensor([dev_s, wall], dtype=torch.float64, device=rdev)
     if world > 1:
@@ -719,7 +752,7 @@ def main():
         cpu, cpu_digest = None, None
         if not args.no_cpu:
             ncpu = w.n if args.cpu_sample <= 0 else min(args.cpu_sample, w.n)
-            rate, dt, nbytes, st = time_cpu_port(w, ncpu, keep_bytes=True)
+            rate, dt, _, st = time_cpu_port(w, ncpu, keep_bytes=True)
             cpu_digest = st.get("ipc_sha256") if ncpu == w.n else None
             cpu = {"value": rate, "unit": "samples/s", "cores": 1, "kind": "port",
                    "sample": "%s batch (%d rows), ingest+flush to IPC bytes in %.1f s, one pass; "
